@@ -234,6 +234,38 @@ def verify_against_oracle(scene_mod, s, adj, rings, runner, res, world):
 
 
 # --------------------------------------------------------------------------------------------------
+# outputs of the timed path, for comparing two builds of the project output for output
+# --------------------------------------------------------------------------------------------------
+DUMP_ROWS = 1 << 18   # at most 7 arrays of 2^18 rows (+ their row positions): about 35 MB per dump
+
+
+def dump_outputs(directory, arrays):
+    """Writes every array as <directory>/<name>.npy, integers as float64 (exact) and floats as float32.  An array with more
+    than DUMP_ROWS rows is replaced by a seeded sample of its rows (the same positions for the same length in every run);
+    the positions go to <name>.rows.npy."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        if len(a) > DUMP_ROWS:
+            rows = np.sort(np.random.default_rng(0).choice(len(a), DUMP_ROWS, replace=False))
+            np.save(os.path.join(directory, f"{name}.rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(directory, f"{name}.npy"), a.astype(np.float64 if a.dtype.kind in "iu" else np.float32))
+
+
+def timed_path_outputs(runner, res, world):
+    """What a caller of the resident path receives after a step: data costs (one GPU: the whole CSR), labels, adjust values."""
+    c = runner.ctx
+    out = {}
+    if world == 1:
+        dc = c.data_costs_download(int(res["dc"].nnz))
+        out.update(data_costs_face_ptr=dc["face_ptr"], data_costs_view=dc["view"], data_costs_cost=dc["cost"])
+    out["labels"] = c.labels_download()
+    seam = c.seam_download(res["seam"])
+    out.update(seam_row_ptr=seam["row_ptr"], seam_row_label=seam["row_label"], seam_x=seam["x"])
+    return out
+
+
+# --------------------------------------------------------------------------------------------------
 def main():
     ap_ = argparse.ArgumentParser()
     ap_.add_argument("--gpus", type=int, default=1)
@@ -251,7 +283,13 @@ def main():
     ap_.add_argument("--with-patches", action="store_true",
                      help="also time texture patches + adjust_colors + local seam leveling (reported under 'extra_stages'; "
                           "never part of the headline metric, which is the three north_star stages)")
+    ap_.add_argument("--dump-outputs", metavar="DIR",
+                     help="write what the last timed step computed (data costs, labels, adjust values) as DIR/<name>.npy; "
+                          "arrays longer than 2^18 rows as a fixed seeded sample of rows; on several GPUs without the data "
+                          "costs, which stay split over the ranks (--impl b200 only)")
     args = ap_.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap_.error("--dump-outputs writes the results of the timed GPU path: use it with --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -342,6 +380,8 @@ def main():
                 "note": "algorithmic bytes per DESIGN.md section 4 (SURVEY 8d); traffic = dram bytes of one "
                         "launch from the ncu --set full capture summarised in profiles/ (C3 workload)"}
     stage_ms = {k: 1e3 * v / 1 for k, v in res["stage_s"].items()}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, timed_path_outputs(runner, res, world))
 
     # ---- parity of the timed run's results at the benchmarked size ---------------------------------
     verify = None

@@ -16,11 +16,15 @@ the smooth scenes lack there too: 37 faces no view sees (label 0) and ten separa
 import ctypes as C
 import os
 import subprocess
+import sys
 
 import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import reference_golden as G  # noqa: E402
+
 CSRC = os.path.join(ROOT, "mvs-texturing_b200", "csrc")
 OUT = os.path.join(ROOT, "tests", "cpp", "_emul")
 CUDA_INC = "/usr/local/cuda/include"
@@ -314,54 +318,20 @@ def test_device_texture_patch_kernels(emul, orc, scene_mod, get_scene, name, adj
 
 def test_device_texture_patches_merge_like_reference_tu(emul, orc, scene_mod, get_scene):
     """Candidate merging (generate_texture_patches.cpp:484-508): label islands whose bounding box lies inside the box of
-    another component of the same label are absorbed.  Crafted on `small` (six one-face islands); compared with the
-    reference's own translation units when libtexref.so is available, else with oracle/patches.py."""
+    another component of the same label are absorbed.  Crafted on `small` (six one-face islands); compared with what the
+    reference's own translation units return on it (tests/golden/reference_tu.json)."""
     import patches as P
     s = get_scene("small")
-    adj = scene_mod.face_adjacency(s.faces)
-    rings = scene_mod.vertex_rings(s.faces, s.verts.shape[0])
-    dc = orc.data_costs(s)
-    labels = orc.view_selection(adj[0], adj[1], dc["face_ptr"], dc["view"], dc["cost"], threads=1)["labels"].copy()
-    ptr = dc["face_ptr"].astype(np.int64)
-    vis = [set((dc["view"][ptr[f]:ptr[f + 1]] + 1).tolist()) for f in range(s.num_faces)]
-    nb = lambda f: [int(a) for a in adj[1][adj[0][f]:adj[0][f + 1]]]
-    islands, used = 0, set()
-    for f in range(s.num_faces):
-        L = labels[f]
-        ring1 = nb(f)
-        if len(ring1) != 3 or any(labels[a] != L for a in ring1):
-            continue
-        ring2 = set(b for a in ring1 for b in nb(a)) - {f} - set(ring1)
-        if any(labels[b] != L for b in ring2) or used & ({f} | set(ring1) | ring2):
-            continue
-        common = set.intersection(*[vis[a] for a in ring1]) - {int(L)}
-        if not common:
-            continue
-        for a in ring1:
-            labels[a] = min(common)          # cut face f off from its component
-        used |= {f} | set(ring1) | ring2
-        islands += 1
-        if islands >= 6:
-            break
+    adj, rings, labels = G.seam_inputs(orc, scene_mod, s)
+    labels, islands = G.island_labels(orc, s, adj, labels)
     assert islands >= 3
     ncomp = sum(len(P.get_subgraphs(adj[0], adj[1], labels, lab)) for lab in range(1, s.num_views + 1))
     ep = _emul_patches(emul, orc, s, adj, labels, None)
     assert len(ep) <= ncomp - islands                          # the islands (at least) were absorbed
-    try:
-        import refpin
-        have_ref = refpin.available()
-    except Exception:
-        have_ref = False
-    if have_ref:
-        rp, _ = refpin.seam_leveling(s, rings, adj, labels, do_global=False)
-        assert len(rp) == len(ep)
-        for a, b in zip(ep, rp):
-            assert _same_patch(a, b.label, b.faces, b.texcoords, b.image, b.validity, b.blending)
-    else:
-        pp, _ = P.generate_texture_patches(orc, s, adj, labels)
-        assert len(pp) == len(ep)
-        for a, q in zip(ep, pp):
-            assert _same_patch(a, q.label, q.faces, q.texcoords, *P.adjust_colors(q, np.zeros((3 * len(q.faces), 3), np.float32)))
+    g = G.load()[0]["texture_patches_with_islands/small"]
+    assert g["islands"] == islands and g["labels"] == [a["label"] for a in ep]
+    for field, d in G.patch_digests(ep, ("faces", "texcoords", "image", "validity", "blending")).items():
+        assert g[field] == d, field
 
 
 def test_patch_plan_merge_chains(emul):
@@ -492,7 +462,7 @@ def test_device_seam_colours_stamping_and_blending_mask(emul, orc, local_inputs,
 @pytest.mark.parametrize("name", ["tiny", "occ", "messy"])
 def test_device_local_seam_leveling(emul, orc, local_inputs, name):
     """Full tex::local_seam_leveling on the device kernels (one batched CG over all patches, on fibers) vs the oracle
-    (scipy splu per patch) and, when libtexref.so is there, vs the reference's own translation units (SparseLU shim):
+    (scipy splu per patch) and vs what the reference's own translation units return (SparseLU shim, tests/golden):
     same validity masks, images within 5e-5 (CG tolerance 1e-5 relative residual; 8-bit quantisation is 4e-3)."""
     import patches as P
     s, adj, rings, labels, seam, pp, pvpi = local_inputs(name)
@@ -508,16 +478,10 @@ def test_device_local_seam_leveling(emul, orc, local_inputs, name):
     print(f"local seam leveling {name}: max |device - oracle| = {worst:.2e}, unknowns {sizes[6]}, CG iterations {sizes[7]}")
     assert worst < 2e-5                                           # the bar of the oracle <-> reference pin
     assert max(float(np.abs(b.image - b0).max()) for b, b0 in zip(pa, before)) > 0.01
-    try:
-        import refpin
-        have_ref = refpin.available()
-    except Exception:
-        have_ref = False
-    if have_ref:
-        rp, _ = refpin.seam_leveling(s, rings, adj, labels, do_global=True, do_local=True)
-        for a, r in zip(ep, [q for q in rp if q.label != 0]):
-            assert np.array_equal(a["validity"], r.validity)
-            assert np.abs(a["image"] - r.image).max() < 5e-5
+    golden = G.load()
+    key = f"local_seam_leveling/{name}"
+    assert golden[0][key]["validity"] == G.patch_digests(ep, ("validity",))["validity"]
+    assert G.image_error(golden, key, [a["image"] for a in ep]) < 5e-5
 
 
 def _random_mrf_problem(rng, n, extra_edges, K, max_labels, unseen_frac=0.03):
@@ -627,31 +591,14 @@ def test_device_multi_gpu_seam_solve_survives_a_dead_peer(emul, orc, scene_mod, 
 
 def test_device_local_seam_leveling_without_global_leveling(emul, orc, local_inputs):
     """texrecon --skip_global_seam_leveling: zero-offset adjust_colors pass (texrecon.cpp:174-183), then local seam leveling on
-    the raw patch colours (larger seam differences to blend away).  Against the reference TUs when available, else the oracle."""
-    import patches as P
+    the raw patch colours (larger seam differences to blend away).  Against what the reference's own translation units
+    return (tests/golden/reference_tu.json)."""
     s, adj, rings, labels, seam, pp, pvpi = local_inputs("tiny")
     ep, sizes = _emul_pipeline(emul, orc, s, adj, labels, None, 2)
-    try:
-        import refpin
-        have_ref = refpin.available()
-    except Exception:
-        have_ref = False
-    if have_ref:
-        rp, _ = refpin.seam_leveling(s, rings, adj, labels, do_global=False, do_local=True)
-        exp = [(q.image, q.validity) for q in rp if q.label != 0]
-    else:
-        pa = []
-        for q in pp:
-            img, val, bl = P.adjust_colors(q, np.zeros((3 * len(q.faces), 3), np.float32))
-            z = P.Patch(q.label, q.faces, q.texcoords, img, q.bbox)
-            z.validity, z.blending = val, bl
-            pa.append(z)
-        P.local_seam_leveling(s, adj, labels, pa, pvpi)
-        exp = [(q.image, q.validity) for q in pa]
-    assert len(ep) == len(exp)
-    for a, (img, val) in zip(ep, exp):
-        assert np.array_equal(a["validity"], val)
-        assert np.abs(a["image"] - img).max() < 1e-4           # raw gain/bias differences are ~10x larger than after global leveling
+    golden = G.load()
+    key = "local_seam_leveling_without_global/tiny"
+    assert golden[0][key]["validity"] == G.patch_digests(ep, ("validity",))["validity"]
+    assert G.image_error(golden, key, [a["image"] for a in ep]) < 1e-4   # raw gain/bias differences are ~10x larger than after global leveling
 
 
 @pytest.mark.parametrize("seed", [0x9E3779B97F4A7C15, 12345])

@@ -1,22 +1,36 @@
 """Pins the oracle against the reference's own translation units.
 
-oracle/_ref/libtexref.so is built from /root/reference/libs/tex/*.cpp (unmodified, compiled where they lie) and
-the dependency shims in oracle/refshim/ (MVE / rayint / Eigen / mapMAP are not vendored in the reference, see
+oracle/_ref/libtexref.so is built from the reference's libs/tex/*.cpp (unmodified, compiled where they lie) and the
+dependency shims in oracle/refshim/ (MVE / rayint / Eigen / mapMAP are not vendored in the reference, see
 oracle/refshim/README.md).  Everything written in libs/tex -- cull rules, projection, validity mask, footprint
 integral, histogram, normalisation -- runs as the reference wrote it; the oracle has to agree bit for bit.
+
+What those translation units return on the inputs below is stored in tests/golden/reference_tu.{json,npz}
+(tests/golden/make_reference_golden.py; format and inputs in tests/golden/reference_golden.py).
 """
+import os
+import sys
+
 import numpy as np
 import pytest
 
-refpin = pytest.importorskip("refpin")
-if not refpin.available():
-    pytest.skip("no libtexref.so and no reference checkout", allow_module_level=True)
+import refpin
+
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+import reference_golden as G  # noqa: E402
+
+D = G.digest
 
 
 @pytest.fixture(scope="module")
 def ref():
-    refpin.lib()
-    return refpin
+    return G.load()
+
+
+def assert_data_costs(g, o):
+    assert int(o["face_ptr"][-1]) == g["nnz"]
+    assert D(o["face_ptr"]) == g["face_ptr"] and D(o["view"]) == g["view"]
+    assert D(o["cost"]) == g["cost"]
 
 
 @pytest.mark.parametrize("name", ["tiny", "small", "occ", "messy"])
@@ -25,28 +39,21 @@ def test_data_costs_match_reference_tu(ref, orc, get_scene, name, data_term):
     """tex::calculate_data_costs (calculate_data_costs.cpp:131-323) vs orc_data_costs: same (face, view) set,
     bit-identical costs."""
     s = get_scene(name)
-    r = ref.data_costs(s, data_term=data_term)
-    o = orc.data_costs(s, data_term=data_term)
-    assert int(r["face_ptr"][-1]) > s.num_faces
-    assert np.array_equal(r["face_ptr"], o["face_ptr"])
-    assert np.array_equal(r["view"], o["view"])
-    assert np.array_equal(r["cost"].view(np.uint32), o["cost"].view(np.uint32))
+    g = ref[0][f"data_costs/{name}/{data_term}"]
+    assert g["nnz"] > s.num_faces
+    assert_data_costs(g, orc.data_costs(s, data_term=data_term))
 
 
 @pytest.mark.parametrize("name", ["tiny", "occ"])
 def test_data_costs_without_visibility_test(ref, orc, get_scene, name):
     s = get_scene(name)
-    r = ref.data_costs(s, visibility=False)
-    o = orc.data_costs(s, visibility=False)
-    assert np.array_equal(r["face_ptr"], o["face_ptr"]) and np.array_equal(r["view"], o["view"])
-    assert np.array_equal(r["cost"].view(np.uint32), o["cost"].view(np.uint32))
-    with_test = ref.data_costs(s)
-    assert int(r["face_ptr"][-1]) >= int(with_test["face_ptr"][-1])
+    g = ref[0][f"data_costs_no_visibility/{name}"]
+    assert_data_costs(g, orc.data_costs(s, visibility=False))
+    with_test = ref[0][f"data_costs/{name}/1"]
+    assert g["nnz"] >= with_test["nnz"]
     if name == "occ":                                                    # floating plates occlude
-        assert int(r["face_ptr"][-1]) > int(with_test["face_ptr"][-1])
-        o2 = orc.data_costs(s)
-        assert np.array_equal(with_test["face_ptr"], o2["face_ptr"]) and np.array_equal(with_test["view"], o2["view"])
-        assert np.array_equal(with_test["cost"].view(np.uint32), o2["cost"].view(np.uint32))
+        assert g["nnz"] > with_test["nnz"]
+        assert_data_costs(with_test, orc.data_costs(s))
 
 
 @pytest.mark.parametrize("mode", [1, 2])
@@ -55,10 +62,10 @@ def test_outlier_removal_matches_reference_tu(ref, orc, get_scene, mode, monkeyp
     before detection depends on the OpenMP merge (:241-249; one thread -> descending view id), the oracle uses
     ascending view id, so sums may differ in the last bits: same survivors, costs within 1e-5."""
     s = get_scene("tiny")
-    r = ref.data_costs(s, outlier_removal=mode)
+    g = ref[0][f"outlier_removal/{mode}"]
     o = orc.data_costs(s, outlier_removal=mode)
-    assert np.array_equal(r["face_ptr"], o["face_ptr"]) and np.array_equal(r["view"], o["view"])
-    assert np.allclose(r["cost"], o["cost"], rtol=0, atol=1e-5)
+    assert int(o["face_ptr"][-1]) == g["nnz"] and D(o["face_ptr"]) == g["face_ptr"] and D(o["view"]) == g["view"]
+    assert np.allclose(ref[1][f"outlier_removal_{mode}_cost"], o["cost"], rtol=0, atol=1e-5)
     base = orc.data_costs(s)
     assert int(o["face_ptr"][-1]) <= int(base["face_ptr"][-1])
 
@@ -66,17 +73,15 @@ def test_outlier_removal_matches_reference_tu(ref, orc, get_scene, mode, monkeyp
 def test_validity_mask_and_erosion_quirk(ref, orc):
     """texture_view.cpp:42-94 (corner flood fill over black pixels) and :109-132 (erosion that leaves the image
     border untouched because the border write lands in the array that is swapped away)."""
-    rng = np.random.RandomState(5)
-    img = rng.randint(1, 255, size=(40, 56, 3)).astype(np.uint8)
-    img[:6, :] = 0; img[:, :4] = 0; img[30:, 50:] = 0          # black frame pieces connected to corners
-    img[15:18, 20:23] = 0                                     # an interior black blob: stays valid
-    m_ref, m_orc = ref.validity_mask(img), orc.validity_mask(img)
+    img, img2 = G.validity_images()
+    m_ref, m_orc = ref[1]["validity_mask"], orc.validity_mask(img)
     assert np.array_equal(m_ref, m_orc) and m_ref[16, 21] == 1 and m_ref[2, 10] == 0
-    e_ref, e_orc = ref.validity_mask(img, erode=True), orc.erode(m_orc)
+    e_ref, e_orc = ref[1]["validity_mask_eroded"], orc.erode(m_orc)
     assert np.array_equal(e_ref, e_orc)
     assert e_ref[6, 10] == 0 and e_ref[7, 10] == 1            # one ring eaten next to the black frame
-    img2 = rng.randint(1, 255, size=(20, 20, 3)).astype(np.uint8)
-    assert ref.validity_mask(img2, erode=True).all()          # the quirk: border pixels stay valid
+    e2_ref = ref[1]["validity_mask_eroded_no_black"]
+    assert e2_ref.all()                                       # the quirk: border pixels stay valid
+    assert np.array_equal(e2_ref, orc.erode(orc.validity_mask(img2)))
 
 
 def test_face_info_matches_reference_tu(ref, orc, get_scene):
@@ -84,24 +89,13 @@ def test_face_info_matches_reference_tu(ref, orc, get_scene):
     (vertex sampling), slivers (slow path / skipped scan lines) and large footprints (fast scan line path)."""
     import ctypes as C
     s = get_scene("small")
-    k = 3
-    rng = np.random.RandomState(11)
-    v, keep = ref._one_view(s, k)
+    k = G.FACE_INFO_VIEW
+    v, keep = refpin._one_view(s, k)
     grad = orc.gradient_magnitude(s.images[k])
-    # triangles around mesh vertices seen by the view: pick faces, then shrink / stretch them
-    dc = orc.data_costs(s)
-    faces = [f for f in range(s.num_faces) if k in dc["view"][int(dc["face_ptr"][f]):int(dc["face_ptr"][f + 1])]]
-    tris = []
-    for f in faces[:300]:
-        t = s.verts[s.faces[f]].astype(np.float32)
-        c = t.mean(axis=0)
-        for scale in (1.0, 0.05, 3.0):
-            tris.append((c + (t - c) * np.float32(scale)).astype(np.float32))
-        sl = t.copy(); sl[2] = (sl[0] + (sl[1] - sl[0]) * np.float32(0.5) + rng.normal(0, 1e-4, 3)).astype(np.float32)
-        tris.append(sl)
-    tris = np.array(tris, np.float32)
+    tris = G.face_info_triangles(s, orc.data_costs(s), k)
     for data_term in (1, 0):
-        q_ref, _ = ref.face_infos(s, k, tris, data_term=data_term)
+        q_ref = ref[1][f"face_quality_{data_term}"]
+        assert len(q_ref) == len(tris)
         q_orc = np.empty(len(tris), np.float32)
         L = orc.lib()
         for i, t in enumerate(tris):
@@ -115,17 +109,16 @@ def test_face_info_matches_reference_tu(ref, orc, get_scene):
 
 def test_tri_and_histogram_match_reference_tu(ref, orc):
     import ctypes as C
-    rng = np.random.RandomState(3)
     L = orc.lib()
-    for _ in range(300):
-        p = rng.uniform(0, 50, size=(3, 2)).astype(np.float32)
-        assert ref.tri_area(*p) == L.orc_tri_area(orc._p(p[0].copy()), orc._p(p[1].copy()), orc._p(p[2].copy()))
-        x, y = rng.uniform(0, 50, size=2).astype(np.float32)
-        assert ref.tri_inside(p[0], p[1], p[2], x, y) == L.orc_tri_inside(orc._p(p[0].copy()), orc._p(p[1].copy()), orc._p(p[2].copy()), C.c_float(x), C.c_float(y))
-    for n in (1, 7, 1000, 200000):
-        v = (rng.gamma(2.0, 3.0, size=n)).astype(np.float32)
+    area, inside = ref[1]["tri_area"], ref[1]["tri_inside"]
+    draws, hist = G.triangle_and_histogram_draws()
+    for i, (p, x, y) in enumerate(draws):
+        assert area[i] == L.orc_tri_area(orc._p(p[0].copy()), orc._p(p[1].copy()), orc._p(p[2].copy()))
+        assert inside[i] == L.orc_tri_inside(orc._p(p[0].copy()), orc._p(p[1].copy()), orc._p(p[2].copy()), C.c_float(x), C.c_float(y))
+    for i, v in enumerate(hist):
+        n = len(v)
         vmax = float(v.max())
-        r = ref.histogram_percentile(v, vmax)
+        r = ref[1]["histogram_percentile"][i]
         o = float(L.orc_histogram_percentile(orc._p(v), C.c_uint64(n), C.c_float(vmax), 10000, C.c_float(0.995)))
         assert r == o
 
@@ -134,13 +127,13 @@ def test_pixel_coords_match_reference_tu(ref, orc, get_scene):
     import ctypes as C
     s = get_scene("tiny")
     L = orc.lib()
-    for k in (0, 5):
-        v, keep = ref._one_view(s, k)
-        for i in range(0, s.verts.shape[0], 37):
+    for j, k in enumerate(G.PIXEL_COORD_VIEWS):
+        v, keep = refpin._one_view(s, k)
+        for n, i in enumerate(G.pixel_coord_vertices(s)):
             x = s.verts[i].copy()
             out = np.empty(2, np.float32)
             L.orc_pixel_coords(C.byref(v), orc._p(x), orc._p(out))
-            assert np.array_equal(ref.pixel_coords(s, k, x).view(np.uint32), out.view(np.uint32))
+            assert np.array_equal(ref[1]["pixel_coords"][j, n].view(np.uint32), out.view(np.uint32))
 
 
 # ---- adjacency graph and MRF model (build_adjacency_graph.cpp, view_selection.cpp) ------------------------------
@@ -149,10 +142,9 @@ def test_adjacency_matches_reference_tu(ref, scene_mod, get_scene, name):
     """tex::build_adjacency_graph (:16-53) on the reference's UniGraph vs scene.face_adjacency (what the oracle and the
     C ABI are fed): same neighbours in the same adjacency-list order, borders (C2s) and separate components (occ) included."""
     s = get_scene(name)
-    rings = scene_mod.vertex_rings(s.faces, s.verts.shape[0])
-    r_ptr, r_idx = ref.build_adjacency(s.faces, s.verts.shape[0], rings)
+    g = ref[0][f"adjacency/{name}"]
     a_ptr, a_idx = scene_mod.face_adjacency(s.faces)
-    assert np.array_equal(r_ptr, a_ptr) and np.array_equal(r_idx, a_idx)
+    assert D(a_ptr) == g["ptr"] and D(a_idx) == g["idx"]
 
 
 @pytest.mark.parametrize("name", ["tiny", "occ"])
@@ -164,31 +156,24 @@ def test_mrf_model_and_label_decoding_match_reference_tu(ref, orc, scene_mod, ge
     s = get_scene(name)
     dc = orc.data_costs(s)
     if name == "tiny":                                           # make a few faces unseen
-        keep = np.ones(len(dc["view"]), bool)
-        ptr = dc["face_ptr"].astype(np.int64)
-        for f in (3, 17, 18, 200):
-            keep[ptr[f]:ptr[f + 1]] = False
-        cnt = np.add.reduceat(keep.astype(np.int64), ptr[:-1]) * (ptr[1:] > ptr[:-1])
-        dc = dict(face_ptr=np.r_[0, np.cumsum(cnt)].astype(np.uint64), view=dc["view"][keep], cost=dc["cost"][keep])
+        dc = G.without_views(dc)
     adj = scene_mod.face_adjacency(s.faces)
-    m = ref.view_selection_model(adj, dc["face_ptr"], dc["view"], dc["cost"], s.num_views)
+    g = ref[0][f"mrf_model/{name}"]
     F = s.num_faces
     ptr = dc["face_ptr"].astype(np.int64)
     seen = ptr[1:] > ptr[:-1]
     assert (~seen).sum() >= (4 if name == "tiny" else 0)
     # edges
     exp = [(i, int(j)) for i in range(F) if seen[i] for j in adj[1][adj[0][i]:adj[0][i + 1]] if i < j and seen[j]]
-    assert [tuple(e) for e in m["edges"].tolist()] == exp
+    edges = np.array(exp, np.uint32).reshape(-1, 2)
+    assert D(edges) == g["edges"]
     # label sets and unaries
-    lp = m["ls_ptr"].astype(np.int64)
-    for f in range(F):
-        ll, lc = m["ls_label"][lp[f]:lp[f + 1]], m["ls_cost"][lp[f]:lp[f + 1]]
-        if seen[f]:
-            assert np.array_equal(ll, dc["view"][ptr[f]:ptr[f + 1]].astype(np.int32) + 1)
-            assert np.array_equal(lc.view(np.uint32), dc["cost"][ptr[f]:ptr[f + 1]].view(np.uint32))
-        else:
-            assert ll.tolist() == [0] and lc.tolist() == [1.0]
-    p = m["params"]
+    ls_label = [dc["view"][ptr[f]:ptr[f + 1]].astype(np.int32) + 1 if seen[f] else np.zeros(1, np.int32) for f in range(F)]
+    ls_cost = [dc["cost"][ptr[f]:ptr[f + 1]] if seen[f] else np.ones(1, np.float32) for f in range(F)]
+    lp = np.r_[0, np.cumsum([len(ll) for ll in ls_label])].astype(np.uint64)
+    ls_label, ls_cost = np.concatenate(ls_label), np.concatenate(ls_cost).astype(np.float32)
+    assert D(lp) == g["ls_ptr"] and D(ls_label) == g["ls_label"] and D(ls_cost) == g["ls_cost"]
+    p = g["params"]
     assert p["potts"] == 1.0 and p["window"] == 5 and abs(p["ratio"] - 0.01) < 1e-12
     assert p["seed"] == 548923723 and p["deterministic"] == 1 and p["model_complete"] == 1 and p["components_updated"] == 1
     assert p["use_multilevel"] == 1 and p["use_spanning_tree"] == 1 and p["use_acyclic"] == 1 and p["force_acyclic"] == 1
@@ -198,16 +183,17 @@ def test_mrf_model_and_label_decoding_match_reference_tu(ref, orc, scene_mod, ge
         if seen[f]:
             c = dc["cost"][ptr[f]:ptr[f + 1]]
             exp_labels[f] = int(dc["view"][ptr[f] + int(np.argmin(c))]) + 1
-    assert np.array_equal(m["labels"], exp_labels)
+    assert D(exp_labels) == g["labels"]
     # the oracle's objective = energy of the recorded model, for the greedy and for the optimised labeling
     o = orc.view_selection(adj[0], adj[1], dc["face_ptr"], dc["view"], dc["cost"], threads=1)
+    lp = lp.astype(np.int64)
     def model_energy(labels):
         e = 0.0
         for f in range(F):
-            ll = m["ls_label"][lp[f]:lp[f + 1]]
+            ll = ls_label[lp[f]:lp[f + 1]]
             k = int(np.flatnonzero(ll == labels[f])[0])
-            e += float(m["ls_cost"][lp[f] + k])
-        e += sum(1.0 for a, b in m["edges"] if labels[a] != labels[b])
+            e += float(ls_cost[lp[f] + k])
+        e += sum(1.0 for a, b in edges if labels[a] != labels[b])
         return e
     for lab in (exp_labels, o["labels"]):
         e_model = model_energy(lab)
@@ -223,11 +209,7 @@ def seam_inputs(orc, scene_mod, get_scene):
     def _get(name):
         if name not in cache:
             s = get_scene(name)
-            adj = scene_mod.face_adjacency(s.faces)
-            rings = scene_mod.vertex_rings(s.faces, s.verts.shape[0])
-            dc = orc.data_costs(s)
-            labels = orc.view_selection(adj[0], adj[1], dc["face_ptr"], dc["view"], dc["cost"], threads=1)["labels"]
-            cache[name] = (s, adj, rings, labels)
+            cache[name] = (s, *G.seam_inputs(orc, scene_mod, s))
         return cache[name]
     return _get
 
@@ -239,22 +221,20 @@ def test_texture_patches_match_reference_tu(ref, orc, seam_inputs, name):
     same patches, faces, bit-identical texcoords, vertex projections, images, validity and blending masks."""
     import patches as P
     s, adj, rings, labels = seam_inputs(name)
-    rp, rvpi = ref.seam_leveling(s, rings, adj, labels, do_global=False)
+    g = ref[0][f"texture_patches/{name}"]                      # label 0 (hole-filling patches, not restated) left out
     pp, pvpi = P.generate_texture_patches(orc, s, adj, labels)
-    rp = [p for p in rp if p.label != 0]                       # label 0 = hole-filling patches (not restated)
-    assert len(rp) == len(pp) >= s.num_views // 2
-    for a, b in zip(rp, pp):
-        assert a.label == b.label and a.faces == b.faces
-        assert np.array_equal(a.texcoords.view(np.uint32), np.asarray(b.texcoords, np.float32).view(np.uint32))
+    assert len(g["labels"]) == len(pp) >= s.num_views // 2
+    for i, b in enumerate(pp):
         img, validity, blending = P.adjust_colors(b, np.zeros((3 * len(b.faces), 3), np.float32))
-        assert np.array_equal(a.validity, validity) and np.array_equal(a.blending, blending)
-        assert np.array_equal(a.image.view(np.uint32), img.view(np.uint32))
-    for v in range(s.verts.shape[0]):
-        mine = {pid: proj for pid, (proj, _f) in pvpi[v].items()}
-        theirs = {pid: xy for pid, xy in rvpi[v].items() if pid < len(pp)}
-        assert set(mine) == set(theirs)
-        for pid in mine:
-            assert np.array_equal(np.asarray(mine[pid], np.float32).view(np.uint32), theirs[pid].view(np.uint32))
+        mine = G.patch_digests([dict(faces=b.faces, texcoords=b.texcoords, image=img, validity=validity, blending=blending)],
+                               ("faces", "texcoords", "validity", "blending", "image"))
+        assert g["labels"][i] == b.label
+        for field, d in mine.items():
+            assert g[field][i] == d[0], field
+    mine = [sorted((pid, np.asarray(proj, np.float32)) for pid, (proj, _f) in pvpi[v].items()) for v in range(s.verts.shape[0])]
+    assert D(np.array([len(m) for m in mine], np.uint32)) == g["projection_count"]
+    assert D(np.array([pid for m in mine for pid, _ in m], np.uint32)) == g["projection_patch"]
+    assert D(np.array([xy for m in mine for _, xy in m], np.float32).reshape(-1, 2)) == g["projection_xy"]
 
 
 @pytest.mark.parametrize("name", ["tiny", "occ", "messy"])
@@ -265,17 +245,16 @@ def test_global_seam_leveling_matches_reference_tu(ref, orc, seam_inputs, name):
     right-hand sides are sampled in patch vs view coordinates, so the adjusted images agree to rounding (2e-5)."""
     import patches as P
     s, adj, rings, labels = seam_inputs(name)
+    g = ref[0][f"global_seam_leveling/{name}"]
     seam = orc.global_seam_leveling(s, rings, labels)
-    rp, _ = ref.seam_leveling(s, rings, adj, labels, do_global=True)
     pp, _ = P.generate_texture_patches(orc, s, adj, labels)
     pa = P.apply_adjust_values(s, pp, seam["row_ptr"], seam["row_label"], seam["x"])
-    rp = [p for p in rp if p.label != 0]
-    assert len(rp) == len(pa)
+    assert len(g["validity"]) == len(pa)
     moved = 0.0
-    for a, b, raw in zip(rp, pa, pp):
-        assert np.array_equal(a.validity, b.validity) and np.array_equal(a.blending, b.blending)
-        assert np.abs(a.image - b.image).max() < 2e-5
-        moved = max(moved, float(np.abs(a.image - raw.image)[a.validity != 0].max()))
+    for i, (b, raw) in enumerate(zip(pa, pp)):
+        assert g["validity"][i] == D(b.validity) and g["blending"][i] == D(b.blending)
+        moved = max(moved, float(np.abs(b.image - raw.image)[b.validity != 0].max()))
+    assert G.image_error(ref, f"global_seam_leveling/{name}", [b.image for b in pa]) < 2e-5
     assert moved > 0.02                                        # the leveling really changed the colours
 
 
@@ -285,17 +264,18 @@ def test_local_seam_leveling_matches_reference_tu(ref, orc, seam_inputs):
     Both solve the same fp32 systems with a direct solver in double (shim elimination / scipy splu): 2e-5."""
     import patches as P
     s, adj, rings, labels = seam_inputs("tiny")
+    g = ref[0]["local_seam_leveling/tiny"]
     seam = orc.global_seam_leveling(s, rings, labels)
-    rp, _ = ref.seam_leveling(s, rings, adj, labels, do_global=True, do_local=True)
     pp, pvpi = P.generate_texture_patches(orc, s, adj, labels)
     pa = P.apply_adjust_values(s, pp, seam["row_ptr"], seam["row_label"], seam["x"])
     before = [p.image.copy() for p in pa]
     P.local_seam_leveling(s, adj, labels, pa, pvpi)
+    assert len(g["validity"]) == len(pa)
     changed = 0.0
-    for a, b, b0 in zip(rp, pa, before):
-        assert np.array_equal(a.validity, b.validity)
-        assert np.abs(a.image - b.image).max() < 2e-5
+    for i, (b, b0) in enumerate(zip(pa, before)):
+        assert g["validity"][i] == D(b.validity)
         changed = max(changed, float(np.abs(b.image - b0).max()))
+    assert G.image_error(ref, "local_seam_leveling/tiny", [b.image for b in pa]) < 2e-5
     assert changed > 0.01
 
 
@@ -303,15 +283,8 @@ def test_adjacency_of_non_manifold_mesh_matches_reference_tu(ref, scene_mod, get
     """An edge shared by three faces (a fin glued onto `tiny`): tex::build_adjacency_graph links all of them; the order of
     the adjacency lists is what scene.face_adjacency has to reproduce (face graphs with degree > 3 take the generic paths of
     the MRF kernels)."""
-    s = get_scene("tiny")
-    verts = np.concatenate([s.verts, (s.verts[s.faces[5]].mean(0) * 1.3)[None].astype(np.float32),
-                            (s.verts[s.faces[40]].mean(0) * 1.3)[None].astype(np.float32)], 0)
-    nv = verts.shape[0]
-    fins = np.array([[s.faces[5][0], s.faces[5][1], nv - 2], [s.faces[5][1], s.faces[5][2], nv - 2],
-                     [s.faces[40][2], s.faces[40][0], nv - 1]], np.uint32)
-    faces = np.ascontiguousarray(np.concatenate([s.faces, fins], 0))
-    rings = scene_mod.vertex_rings(faces, nv)
-    r_ptr, r_idx = ref.build_adjacency(faces, nv, rings)
+    verts, faces = G.mesh_with_fins(get_scene("tiny"))
+    g = ref[0]["adjacency/tiny_with_fins"]
     a_ptr, a_idx = scene_mod.face_adjacency(faces)
-    assert int(np.diff(r_ptr).max()) > 3
-    assert np.array_equal(r_ptr, a_ptr) and np.array_equal(r_idx, a_idx)
+    assert g["max_degree"] > 3
+    assert D(a_ptr) == g["ptr"] and D(a_idx) == g["idx"]
